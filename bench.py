@@ -70,7 +70,12 @@ def parse():
     ap.add_argument("--profile-waves", type=int, default=200, help="waves timed individually for the roofline line")
     ap.add_argument("--arena-words", type=int, default=0)
     ap.add_argument("--kwave-capture", action="store_true", help="ncu helper: play --warmup plies (deep trees), then run --profile-waves eager waves and exit")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed plies, write what the last one returned (rank 0) as DIR/<name>.npy, float32 / float64, <= 64 MB")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be >= 1")
+    return a
 
 
 # ---------------------------------------------------------------------------------------------
@@ -339,7 +344,7 @@ class Runner:
         tot_exp, tot_launch, games_done, tuples_done = [float(x) for x in n]
         return dict(dev_ms=dev_ms, e2e_ms=e2e_ms, wall_ms=wall_ms, expansions=tot_exp, launches=tot_launch, games_done=games_done,
                     tuples_done=tuples_done, waves=sp.waves - waves0, steps=steps, c0=c0, c1=c1, clocks=clk,
-                    value=tot_exp / (dev_ms * 1e-3), e2e=tot_exp / (e2e_ms * 1e-3))
+                    value=tot_exp / (dev_ms * 1e-3), e2e=tot_exp / (e2e_ms * 1e-3), last=out)
 
     def kwave_roofline(self, n_waves):
         """k_wave timed per launch with CUDA events on the launching stream, in situ (the trees are those of the plies played so far)."""
@@ -547,6 +552,37 @@ def leg_soak(runner, plies):
                 note="seed-0 (untrained) network: games end by king capture or the 60-ply no-capture rule (main.py:1532-1545)")
 
 
+def dump_outputs(d, out, limit=63 << 20):
+    """Writes what SelfPlay.step() returned (`out`) as d/<name>.npy: per game slot the chosen child, its win rate (mcts.Q) and the
+    game status after the move; per game that ended in this ply its slot, length, z and dense pi rows (the (s, pi, z) tuples of
+    selfplay(), game after game).  Integers are stored exactly as float64.  game_slots.npy names the slots written: all of them,
+    or, when that would exceed `limit` bytes (64 MB less room for the .npy headers), a fixed seeded sample."""
+    st = out["status"]
+    per_game = dict(choice=out["choice"].astype(np.float64), win_rate=out["win_rate"].astype(np.float32),
+                    boards=st["boards"].astype(np.float32), side=st["side"].astype(np.float64), terminal=st["terminal"].astype(np.float64),
+                    winner=st["winner"].astype(np.float64), ply=st["ply"].astype(np.float64), rr=st["rr"].astype(np.float64),
+                    q=st["q"].astype(np.float32), root_N=st["root_N"].astype(np.float64))
+    B = len(out["choice"])
+    fin = {g: (rec.z.astype(np.float64), rec.dense_pi()) for g, rec in out["finished"]}
+    cost = np.full(B, sum(v[0].nbytes for v in per_game.values()), dtype=np.int64)
+    for g, (z, pi) in fin.items():
+        cost[g] += 16 + z.nbytes + pi.nbytes
+    if cost.sum() <= limit:
+        slots = np.arange(B)
+    else:
+        order = np.random.RandomState(0).permutation(B)
+        slots = np.sort(order[:int(np.searchsorted(np.cumsum(cost[order]), limit, side="right"))])
+    done = [g for g in slots if g in fin]
+    arrays = {k: v[slots] for k, v in per_game.items()}
+    arrays.update(game_slots=slots.astype(np.float64), finished_slot=np.array(done, dtype=np.float64),
+                  finished_plies=np.array([len(fin[g][0]) for g in done], dtype=np.float64),
+                  finished_z=np.concatenate([fin[g][0] for g in done] or [np.zeros(0)]),
+                  finished_pi=np.concatenate([fin[g][1] for g in done] or [np.zeros((0, 2086))]))
+    os.makedirs(d, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(d, k + ".npy"), v)
+
+
 # ---------------------------------------------------------------------------------------------
 def run_ours(a, rank, world, local_rank):
     import torch.distributed as dist
@@ -565,6 +601,8 @@ def run_ours(a, rank, world, local_rank):
 
     clocks = ClockSampler(local_rank) if rank == 0 else None
     m = main.plies(a.steps, a.warmup, clocks=clocks)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, m["last"])
     roof = main.kwave_roofline(a.profile_waves) if rank == 0 else None
     if world > 1:
         dist.barrier()

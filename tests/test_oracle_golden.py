@@ -213,27 +213,16 @@ def test_fifo_schedule_spec_with_playouts_that_end_in_their_first_step():
 
 
 def test_deterministic_event_loop_runs_the_reference_coroutines_to_the_same_trees():
-    """oracle/detloop.py: the UNMODIFIED coroutines of the reference (tree_search / start_tree_search / prediction_worker) on a
-    deterministic event loop give the visit counts of the real uvloop run AND of the C restatement.  Needs the reference (live or
-    staged)."""
-    import os
-    import sys
-    from conftest import ROOT
-    sys.path.insert(0, os.path.join(ROOT, "oracle"))
-    import stage_reference as S
-    if S.staged_dir() is None:
-        pytest.skip("reference not present")
-    import detloop as D
-    import ref_harness as H
-    from conftest import load_golden
-    d = load_golden("k16_stats.json.gz")
-    for r in d["records"][:12]:
-        ref, t, loop = D.make_tree(H, H.FAKE_NETS[d["net"]], 16, r["state"], "busy")
-        with np.errstate(all="ignore"):
-            D.run_reference_search(ref, t, r["state"], r["player"], r["rr"], d["playouts"], loop)
-        loop.close()
-        v = [int(c.N) for c in t.root.child.values()]
-        assert v == r["k16"] or v == r["k16_delay2ms"]
+    """The UNMODIFIED coroutines of the reference (tree_search / start_tree_search / prediction_worker) on oracle/detloop.py's
+    deterministic event loop (tests/golden/k16_detloop.json, oracle/gen_golden_detloop.py) give the visit counts of the real uvloop
+    run AND of the C restatement."""
+    d = load_golden("k16_detloop.json")["positions"]
+    real = load_golden("k16_stats.json.gz")
+    assert d["net"] == real["net"] and d["playouts"] == real["playouts"] and len(d["records"]) == 12
+    for r, u in zip(d["records"], real["records"]):
+        assert (r["state"], r["player"], r["rr"]) == (u["state"], u["player"], u["rr"])
+        v = r["visits"]
+        assert v == u["k16"] or v == u["k16_delay2ms"]
         o = O.Tree(O.from_state(r["state"]))
         o.search_fifo(0 if r["player"] == "w" else 1, r["rr"], d["playouts"], 16, d["net"])
         assert v == [int(x) for x in o.root_children()[1]]
@@ -242,43 +231,22 @@ def test_deterministic_event_loop_runs_the_reference_coroutines_to_the_same_tree
 def test_fifo_schedule_across_tree_reuse_matches_the_reference_coroutines():
     """Several consecutive searches at search_threads=16 with MCTS_tree.update_tree in between (the self-play / play-mode pattern):
     the stored Q, the left-over visit counts of the re-used subtree and the frozen root N must carry over exactly as in the
-    reference's object tree.  Reference side: its own coroutines on the deterministic loop; other side: the C restatement."""
-    import os
-    import sys
-    from conftest import ROOT
-    sys.path.insert(0, os.path.join(ROOT, "oracle"))
-    import stage_reference as S
-    if S.staged_dir() is None:
-        pytest.skip("reference not present")
-    import detloop as D
-    import ref_harness as H
-    ref = H.load_reference()
-    net, P = "hash_pos", 96
-    state, player, rr = O.START, "w", 0
-    rtree = None
+    reference's object tree.  Reference side: its own coroutines on the deterministic loop (tests/golden/k16_detloop.json);
+    other side: the C restatement."""
+    d = load_golden("k16_detloop.json")["tree_reuse"]
+    net, P = d["net"], d["playouts"]
+    board, player, rr = O.from_state(O.START), "w", 0
     ctree = O.Tree()
-    for ply in range(5):
-        loop = D.DetLoop("busy")
-        import asyncio
-        asyncio.set_event_loop(loop)
-        if rtree is None:
-            rtree = ref.MCTS_tree_py312(state, H.FAKE_NETS[net], 16)
-        rtree.loop = loop
-        rtree.sem = asyncio.Semaphore(16)                 # fresh primitives for the fresh loop (main() builds new coroutines each call)
-        rtree.queue = asyncio.Queue(16)
-        rtree.running_simulation_num = 0
-        with np.errstate(all="ignore"):
-            D.run_reference_search(ref, rtree, state, player, rr, P, loop)
-        loop.close()
+    assert len(d["plies"]) == 5
+    for ply, g in enumerate(d["plies"]):
+        assert (O.to_state(board), player, rr) == (g["state"], g["player"], g["rr"]), ply
         assert ctree.search_fifo(0 if player == "w" else 1, rr, P, 16, net) == 0
         mv, N, W, Pp, Q = ctree.root_children()
-        got = [(a, int(c.N), H.f32_bits(c.Q)) for a, c in rtree.root.child.items()]
-        want = [(O.move_str(m), int(n), H.f32_bits(q)) for m, n, q in zip(mv, N, Q)]
+        got = [tuple(c) for c in g["children"]]
+        want = [(O.move_str(m), int(n), bits(q)) for m, n, q in zip(mv, N, Q)]
         assert got == want, ply
         best = int(np.argmax(N))
-        act = O.move_str(mv[best])
-        nxt = ref.GameBoard.sim_do_action(act, state)
-        rr = rr + 1 if ref.is_kill_move(state, nxt) == 0 else 0
-        rtree.update_tree(act)
+        board, cap = O.apply_move(board, mv[best])
+        rr = rr + 1 if cap == 0 else 0
         ctree.update(best)
-        state, player = nxt, ("b" if player == "w" else "w")
+        player = "b" if player == "w" else "w"
