@@ -8,7 +8,8 @@ LIB_PATH = os.path.join(_HERE, "libcchess_b200.so")
 
 NSQ, NLABEL, MAXCHILD, ENC_LEN, STATUS_BYTES, MT_WORDS = 90, 2086, 128, 1260, 112, 626
 F32, BF16, F16, BOARD = 0, 1, 2, 3
-ERR_NAMES = {1: "NOMOVES", 2: "NOLABEL", 4: "DEPTH", 8: "ARENA", 16: "CHILDREN"}
+ERR_NAMES = {1: "NOMOVES", 2: "NOLABEL", 4: "DEPTH", 8: "ARENA", 16: "CHILDREN", 32: "NOCHILD"}
+NOMOVE = 0xFFFF
 
 _lib = None
 
@@ -50,6 +51,7 @@ def _sig(L):
     L.cz_engine_root_keys.argtypes = [vp, vp, vp]
     L.cz_engine_play_status.argtypes = [vp, vp, vp, vp]
     L.cz_engine_status_packed.argtypes = [vp, vp, vp]
+    L.cz_engine_play_moves.argtypes = [vp, vp, vp, vp]
     L.cz_engine_unfinished.argtypes = [vp, vp, vp]
     L.cz_engine_unfinished_async.argtypes = [vp, vp, vp]
     L.cz_engine_root_children.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp]

@@ -1155,15 +1155,9 @@ __device__ __forceinline__ void copy_block(uint32_t *__restrict__ dst, const uin
     }
 }
 
-__global__ void __launch_bounds__(32 * WARPS_PER_BLOCK) k_play(Dev E) {
-    const int lane = threadIdx.x & 31, g = blockIdx.x * WARPS_PER_BLOCK + (threadIdx.x >> 5);
-    if (g >= E.B) return;
-    uint32_t *h = E.hdr + (size_t)g * HW;
-    uint8_t *b = E.root_board + (size_t)g * 96;
-    const int choice = E.st_choice[g];
-    if (choice < 0) { write_status(E, g, h, b, 0.0f, lane); return; }
-    const int rcnt = (int)h[H_ROOTCNT];
-    if (rcnt <= 0 || choice >= rcnt) { if (lane == 0) atomicOr(h + H_ERR, CZ_ERR_NOMOVES); write_status(E, g, h, b, 0.0f, lane); return; }
+// Plays root child `choice` (0 <= choice < rcnt = the root's child count) of game g: the whole of update_tree + the board update,
+// shared by k_play (child index) and k_play_moves (move code).
+__device__ __forceinline__ void play_child(const Dev &E, int g, uint32_t *h, uint8_t *b, int choice, int rcnt, int lane) {
     const uint32_t flags = h[H_FLAGS];
     const int cur = (flags & F_CUR) ? 1 : 0;
     const uint32_t *old = arena_half(E, g, cur);
@@ -1242,6 +1236,44 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK) k_play(Dev E) {
     }
     __syncwarp();
     write_status(E, g, h, b, q, lane);
+}
+
+__global__ void __launch_bounds__(32 * WARPS_PER_BLOCK) k_play(Dev E) {
+    const int lane = threadIdx.x & 31, g = blockIdx.x * WARPS_PER_BLOCK + (threadIdx.x >> 5);
+    if (g >= E.B) return;
+    uint32_t *h = E.hdr + (size_t)g * HW;
+    uint8_t *b = E.root_board + (size_t)g * 96;
+    const int choice = E.st_choice[g];
+    if (choice < 0) { write_status(E, g, h, b, 0.0f, lane); return; }
+    const int rcnt = (int)h[H_ROOTCNT];
+    if (rcnt <= 0 || choice >= rcnt) { if (lane == 0) atomicOr(h + H_ERR, CZ_ERR_NOMOVES); write_status(E, g, h, b, 0.0f, lane); return; }
+    play_child(E, g, h, b, choice, rcnt, lane);
+}
+
+// update_tree(act) keyed by the move (main.py:272-276): the root child whose META move equals st_choice[g] (CZ_NOMOVE = leave the
+// game alone) is found by a lane-parallel scan of the root block, first match by ballot, and played as k_play plays it.  A move
+// that is not a child -- or any move at an unexpanded root -- raises CZ_ERR_NOCHILD (the reference's KeyError) and leaves the game
+// untouched; its status record is written either way.
+__global__ void __launch_bounds__(32 * WARPS_PER_BLOCK) k_play_moves(Dev E) {
+    const int lane = threadIdx.x & 31, g = blockIdx.x * WARPS_PER_BLOCK + (threadIdx.x >> 5);
+    if (g >= E.B) return;
+    uint32_t *h = E.hdr + (size_t)g * HW;
+    uint8_t *b = E.root_board + (size_t)g * 96;
+    const uint32_t mv = (uint32_t)E.st_choice[g];
+    if (mv == CZ_NOMOVE) { write_status(E, g, h, b, 0.0f, lane); return; }
+    const int rcnt = (int)h[H_ROOTCNT];
+    int choice = -1;
+    if (rcnt > 0) {
+        const uint32_t rcs = (uint32_t)((rcnt + 7) & ~7);
+        const uint32_t *meta = arena_half(E, g, (h[H_FLAGS] & F_CUR) ? 1 : 0) + h[H_ROOTBASE] + HDR + 3 * rcs;
+        for (int i0 = 0; i0 < rcnt && choice < 0; i0 += 32) {          // (choice is warp-uniform: it comes from a ballot)
+            const int i = i0 + lane;
+            const unsigned m = __ballot_sync(CZ_FULL, i < rcnt && (meta[i] & 0xFFFFu) == mv);
+            if (m) choice = i0 + __ffs(m) - 1;
+        }
+    }
+    if (choice < 0) { if (lane == 0) atomicOr(h + H_ERR, CZ_ERR_NOCHILD); write_status(E, g, h, b, 0.0f, lane); return; }
+    play_child(E, g, h, b, choice, rcnt, lane);
 }
 
 // ---- stateless batched rules ------------------------------------------------------------
@@ -1796,6 +1828,21 @@ int cz_engine_play_status(cz_engine *e, void *stream, const int32_t *child_index
 }
 
 int cz_engine_play(cz_engine *e, void *stream, const int32_t *child_index) { return cz_engine_play_status(e, stream, child_index, nullptr); }
+
+int cz_engine_play_moves(cz_engine *e, void *stream, const uint16_t *moves, uint8_t *status) {
+    if (!e || !moves) return fail(CZ_EINVAL, "cz_engine_play_moves: null");
+    cudaStream_t st = (cudaStream_t)stream;
+    const size_t B = (size_t)e->d.B;
+    CUDA_TRY(cudaSetDevice(e->device));
+    for (size_t g = 0; g < B; g++) e->h_choice[g] = (int32_t)moves[g];     // the move codes travel in the child-index buffer
+    CUDA_TRY(cudaMemcpyAsync(e->d.st_choice, e->h_choice, B * 4, cudaMemcpyHostToDevice, st));
+    k_play_moves<<<nblk(e->d.B, WARPS_PER_BLOCK), 32 * WARPS_PER_BLOCK, 0, st>>>(e->d);
+    CUDA_TRY(cudaGetLastError());
+    if (status) CUDA_TRY(cudaMemcpyAsync(e->h_status, e->d.st_status, B * CZ_STATUS_BYTES, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));   // h_choice is reused by the next call
+    if (status) memcpy(status, e->h_status, B * CZ_STATUS_BYTES);
+    return CZ_OK;
+}
 
 int cz_engine_status_packed(cz_engine *e, void *stream, uint8_t *status) {
     if (!e || !status) return fail(CZ_EINVAL, "cz_engine_status_packed: null");

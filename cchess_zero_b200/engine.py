@@ -155,6 +155,21 @@ class Engine:
         check(lib().cz_engine_play_status(self.h, _stream(), _hp(ci), _hp(rec)), "cz_engine_play_status")
         return self._unpack_status(rec) if want_status else None
 
+    def play_moves(self, moves, want_status=True):
+        """update_tree(act) keyed by the move code (src | dst << 7) + the board update for every game with moves[g] != NOMOVE:
+        the tree follows a move chosen elsewhere (the opponent's, human_move main.py:1394-1430).  status()["q"] is Q(act) of this
+        tree.  A move that is not a child of an expanded root leaves that game untouched and flags it with NOCHILD; with
+        want_status the flag raises EngineError (the reference's KeyError, main.py:275)."""
+        mv = np.ascontiguousarray(moves, dtype=np.uint16)
+        assert mv.shape == (self.B,)
+        self.launches += 1
+        rec = np.zeros((self.B, STATUS_BYTES), dtype=np.uint8) if want_status else None
+        check(lib().cz_engine_play_moves(self.h, _stream(), _hp(mv), _hp(rec)), "cz_engine_play_moves")
+        if not want_status:
+            return None
+        self.raise_on_error()
+        return self._unpack_status(rec)
+
     @staticmethod
     def _unpack_status(rec):
         tail = np.ascontiguousarray(rec[:, 96:112]).view(np.int32)

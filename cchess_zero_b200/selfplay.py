@@ -157,6 +157,44 @@ class GameRecord:
         return zip(self.states, self.dense_pi(), self.z)
 
 
+def choose_moves(n_children, visits, live, mt, exploration, temperature, n_threads=1):
+    """get_action's move choice (main.py:1339-1348) for every game with live[g]: the index into the root's children drawn from
+    softmax(1/T * log(visits)), with the reference's Dirichlet noise when `exploration`.  mt [B][MT_WORDS]: one legacy MT19937
+    state per game, advanced in place exactly as numpy's RandomState would be.  -1 for the other games."""
+    B = len(n_children)
+    choice = np.full(B, -1, dtype=np.int32)
+    with np.errstate(divide="ignore", invalid="ignore"):
+        # softmax(1/T * log(visits)) of main.py:1341, 1111-1116.  log / exp / max are element-wise or exact, so they are
+        # taken over the whole [B,128] batch at once (padding: visits 0 -> -inf -> exp 0); the order-sensitive row sum, the
+        # Dirichlet / choice draws and the cumulative sums happen per game in csrc/cz_host.cu, operation for operation what
+        # numpy does for `probs /= np.sum(probs)`, RandomState.dirichlet and RandomState.choice (main.py:1345-1348).
+        lv = (1.0 / temperature) * np.log(visits.astype(np.int64))
+        valid = np.arange(MAXCHILD)[None, :] < n_children[:, None]
+        lv[~valid] = -np.inf
+        ex = np.ascontiguousarray(np.exp(lv - np.max(lv, axis=1, keepdims=True)))
+    probs = np.empty((B, MAXCHILD), dtype=np.float64)
+    fallback = np.zeros(B, dtype=np.uint8)
+    live8 = np.ascontiguousarray(live, dtype=np.uint8)
+    nn = np.ascontiguousarray(n_children, dtype=np.int32)
+    from ._lib import lib
+    import ctypes as C
+    vp = lambda a: a.ctypes.data_as(C.c_void_p)  # noqa: E731
+    rcode = lib().cz_host_choose_moves(B, vp(live8), vp(nn), vp(ex), 1 if exploration else 0, vp(mt), vp(choice), vp(probs),
+                                       vp(fallback), n_threads)
+    if rcode:
+        raise EngineError("cz_host_choose_moves failed (%d)" % rcode)
+    for g in np.nonzero(fallback)[0]:
+        # a probability vector numpy would reject (NaN priors ...): let numpy raise exactly what the reference would raise
+        n = int(nn[g])
+        rs = np.random.RandomState()
+        rs.set_state(("MT19937", mt[g, :624].copy(), int(mt[g, 624]), 0, 0.0))
+        pr = ex[g, :n] / np.sum(ex[g, :n])
+        choice[g] = int(rs.choice(n, p=pr))          # (the Dirichlet draws were consumed by the native sampler, as in the reference)
+        st_ = rs.get_state()
+        mt[g, :624], mt[g, 624] = st_[1], st_[2]
+    return choice
+
+
 class _Lane:
     """One half-batch of a pipelined SelfPlay: its own engine, I/O buffers and evaluator scratch."""
 
@@ -354,12 +392,12 @@ class SelfPlay:
             cs.wait_stream(side)
         self.graph = g
 
-    def _search_pipeline(self):
+    def _search_pipeline(self, sel):
         e = self.engine
         A, Bn = self.lanes
-        for p in np.unique(self.playouts[self.live]):
-            e.begin_search(int(p), (self.live & (self.playouts == p)).astype(np.uint8))
-        pmax = int(self.playouts[self.live].max()) if self.live.any() else 0
+        for p in np.unique(self.playouts[sel]):
+            e.begin_search(int(p), (sel & (self.playouts == p)).astype(np.uint8))
+        pmax = int(self.playouts[sel].max()) if sel.any() else 0
         A.engine.wave(A.nn_in, A.logits, A.value)      # prologue: lane A's first leaves
         waves = 1
         while True:
@@ -415,13 +453,13 @@ class SelfPlay:
             self._bucket_graphs[n] = g
         g.replay()
 
-    def _search_compact(self):
+    def _search_compact(self, sel):
         e = self.engine
         if self.plan is not None and hasattr(self.plan, "refresh_if_stale"):
             self.plan.refresh_if_stale()
-        for p in np.unique(self.playouts[self.live]):
-            e.begin_search(int(p), (self.live & (self.playouts == p)).astype(np.uint8))
-        pmax = int(self.playouts[self.live].max()) if self.live.any() else 0
+        for p in np.unique(self.playouts[sel]):
+            e.begin_search(int(p), (sel & (self.playouts == p)).astype(np.uint8))
+        pmax = int(self.playouts[sel].max()) if sel.any() else 0
         waves = 0
         while True:
             e.wave_compact(self.nn_stage, self.nn_in, self.logits, self.value)
@@ -458,18 +496,19 @@ class SelfPlay:
             self._eval(self.nn_in)
         self.graph = g
 
-    def search(self):
-        """MCTS_tree.main for every live game: `playouts[g]` playouts each."""
+    def search(self, mask=None):
+        """MCTS_tree.main for every live game (mask: only those live games with mask[g]): `playouts[g]` playouts each."""
+        sel = self.live if mask is None else self.live & np.asarray(mask, dtype=bool)
         if self.lanes is not None:
-            return self._search_pipeline()
+            return self._search_pipeline(sel)
         if self.compact:
-            return self._search_compact()
+            return self._search_compact(sel)
         e = self.engine
         if self.plan is not None and hasattr(self.plan, "refresh_if_stale"):
             self.plan.refresh_if_stale()       # weights trained / restored since the last search (the graph reads them in place)
-        for p in np.unique(self.playouts[self.live]):
-            e.begin_search(int(p), (self.live & (self.playouts == p)).astype(np.uint8))
-        pmax = int(self.playouts[self.live].max()) if self.live.any() else 0
+        for p in np.unique(self.playouts[sel]):
+            e.begin_search(int(p), (sel & (self.playouts == p)).astype(np.uint8))
+        pmax = int(self.playouts[sel].max()) if sel.any() else 0
         waves = 0
         while True:
             if self.graph is not None:
@@ -493,40 +532,12 @@ class SelfPlay:
         e = self.engine
         self.search()
         rc = e.root_children(want_wpq=False)                      # n, moves, visits: what get_action reads (main.py:1339)
-        choice = np.full(self.B, -1, dtype=np.int32)
         live = np.nonzero(self.live)[0]
         if (rc["n"][live] <= 0).any():
             e.raise_on_error()
             raise EngineError("game %d has no root children" % int(live[np.argmax(rc["n"][live] <= 0)]))
-        with np.errstate(divide="ignore", invalid="ignore"):
-            # softmax(1/T * log(visits)) of main.py:1341, 1111-1116.  log / exp / max are element-wise or exact, so they are
-            # taken over the whole [B,128] batch at once (padding: visits 0 -> -inf -> exp 0); the order-sensitive row sum, the
-            # Dirichlet / choice draws and the cumulative sums happen per game in csrc/cz_host.cu, operation for operation what
-            # numpy does for `probs /= np.sum(probs)`, RandomState.dirichlet and RandomState.choice (main.py:1345-1348).
-            lv = (1.0 / self.temperature) * np.log(rc["visits"].astype(np.int64))
-            valid = np.arange(MAXCHILD)[None, :] < rc["n"][:, None]
-            lv[~valid] = -np.inf
-            ex = np.ascontiguousarray(np.exp(lv - np.max(lv, axis=1, keepdims=True)))
-        probs = np.empty((self.B, MAXCHILD), dtype=np.float64)
-        fallback = np.zeros(self.B, dtype=np.uint8)
-        live8 = np.ascontiguousarray(self.live, dtype=np.uint8)
         nn = np.ascontiguousarray(rc["n"], dtype=np.int32)
-        from ._lib import lib
-        import ctypes as C
-        vp = lambda a: a.ctypes.data_as(C.c_void_p)  # noqa: E731
-        rcode = lib().cz_host_choose_moves(self.B, vp(live8), vp(nn), vp(ex), 1 if self.exploration else 0, vp(self._mt), vp(choice), vp(probs),
-                                           vp(fallback), self._threads)
-        if rcode:
-            raise EngineError("cz_host_choose_moves failed (%d)" % rcode)
-        for g in np.nonzero(fallback)[0]:
-            # a probability vector numpy would reject (NaN priors ...): let numpy raise exactly what the reference would raise
-            n = int(rc["n"][g])
-            rs = np.random.RandomState()
-            rs.set_state(("MT19937", self._mt[g, :624].copy(), int(self._mt[g, 624]), 0, 0.0))
-            pr = ex[g, :n] / np.sum(ex[g, :n])
-            choice[g] = int(rs.choice(n, p=pr))          # (the Dirichlet draws were consumed by the native sampler, as in the reference)
-            st_ = rs.get_state()
-            self._mt[g, :624], self._mt[g, 624] = st_[1], st_[2]
+        choice = choose_moves(nn, rc["visits"], self.live, self._mt, self.exploration, self.temperature, self._threads)
         if self.keep_records:
             entry = dict(boards=self.boards, n=nn, moves=rc["moves"], visits=rc["visits"], choice=choice)
             for g in live:
@@ -696,6 +707,17 @@ class cchess_main(object):
         self.data_buffer, extra = load_replay(path)
         self.lr_multiplier = extra.get("lr_multiplier", self.lr_multiplier)
         self.global_step = extra.get("global_step", self.global_step)
+
+    def policy_evaluate(self, opponent, n_games=10):
+        """main.py:1207-1222 (commented out in the reference): n_games matches of this object's network against `opponent` (a
+        cchess_main or a network), colours alternating, both sides with this object's playout_counts / search_threads, played
+        concurrently by arena.Arena.  Returns the reference's win_ratio = (win + 0.5 * tie) / n_games."""
+        from .arena import Arena
+        opp = getattr(opponent, "policy_value_netowrk", opponent)
+        s = Arena(self.policy_value_netowrk, opp, n_games, self.playout_counts, search_threads_a=self.search_threads,
+                  temperature=self.temperature).play().summary()
+        print("num_playouts:{}, win: {}, lose: {}, tie:{}".format(self.playout_counts, s["w"], s["l"], s["d"]))
+        return s["win_ratio"]
 
     def run(self, max_batches=None):  # main.py:1224-1248
         batch_iter = 0

@@ -50,6 +50,7 @@ extern "C" {
 #define CZ_ERR_DEPTH 4       /* search path deeper than the path stack */
 #define CZ_ERR_ARENA 8       /* tree arena exhausted */
 #define CZ_ERR_CHILDREN 16   /* more than CZ_MAXCHILD moves */
+#define CZ_ERR_NOCHILD 32    /* move is not a child of an expanded root (reference: KeyError in update_tree, main.py:275) */
 
 const char *cz_last_error(void);
 int cz_version(void);
@@ -173,6 +174,12 @@ int cz_engine_play(cz_engine *e, void *stream, const int32_t *child_index /* [B]
 #define CZ_STATUS_BYTES 112
 int cz_engine_play_status(cz_engine *e, void *stream, const int32_t *child_index /* [B] */, uint8_t *status /* host [B][112] or NULL */);
 int cz_engine_status_packed(cz_engine *e, void *stream, uint8_t *status /* host [B][112] */);
+/* MCTS_tree.update_tree(act) keyed by the MOVE (main.py:272-276, as human_move calls it at 1418) + the board update: for every game
+ * the root child whose move equals moves[g] is played exactly as cz_engine_play_status plays its index; the status record's Q is
+ * Q(act) of THIS tree (human_move's win_rate).  moves[g] == CZ_NOMOVE leaves game g alone.  A move that is not a child of the root,
+ * or any move at a root that was never expanded, sets CZ_ERR_NOCHILD on that game and leaves it untouched (status still written). */
+#define CZ_NOMOVE 0xFFFF
+int cz_engine_play_moves(cz_engine *e, void *stream, const uint16_t *moves /* host [B] */, uint8_t *status /* host [B][112] or NULL */);
 
 /* Game status (cchess_main.check_end main.py:1380-1392): HOST buffers, any may be NULL; synchronises.
  * terminal: 0 running, 1 king captured, 2 draw (restrict_round >= 60); winner: 0 'w', 1 'b', -1 none. */
